@@ -11,6 +11,7 @@ binning -> tile blend (+ the NCCL frame gather when N > 1).
   python bench.py --gpus N --steps K --warmup W            # this repo (CUDA, through the C ABI)
   python bench.py --impl reference --steps K --warmup W    # the reference's path on the host CPU
                                                            # (oracle port: the reference cannot be built here)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's frames to DIR/*.npy
 Prints ONE JSON line on rank 0.
 """
 from __future__ import annotations
@@ -133,6 +134,36 @@ def make_cloud(n: int):
     return B.random_gaussians_3d_seeded(n, 0)
 
 
+def read_device(ptr: int, nbytes: int) -> np.ndarray:
+    """Device memory -> host bytes through the driver API (synchronous; the caller has synchronised the producers)."""
+    import ctypes as C
+
+    got = np.empty(nbytes, np.uint8)
+    cu = C.CDLL("libcuda.so.1")
+    cu.cuMemcpyDtoH_v2.argtypes = [C.c_void_p, C.c_uint64, C.c_size_t]
+    assert cu.cuMemcpyDtoH_v2(got.ctypes.data_as(C.c_void_p), C.c_uint64(ptr), got.size) == 0
+    return got
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_frames(out_dir: str, frames: np.ndarray) -> None:
+    """--dump-outputs: the (views, H, W, 4) RGBA8 frames of the last timed step as float32 .npy files, so that two builds
+    can be compared output for output.  Frames larger than DUMP_LIMIT_BYTES in float32 (more than two 1080p views) are
+    replaced by the same seeded sample of pixel positions in every view: frames_sample.npy (views, P, 4) and
+    frames_sample_pixel.npy (P,), the row-major pixel indices as float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    v, h, w, c = frames.shape
+    if frames.size * 4 <= DUMP_LIMIT_BYTES:
+        np.save(os.path.join(out_dir, "frames.npy"), frames.astype(np.float32))
+        return
+    p = (DUMP_LIMIT_BYTES - 4096) // (4 * v * c + 8)        # (4 KB for the two .npy headers)
+    pix = np.sort(np.random.default_rng(0).choice(h * w, p, replace=False))
+    np.save(os.path.join(out_dir, "frames_sample.npy"), frames.reshape(v, h * w, c)[:, pix].astype(np.float32))
+    np.save(os.path.join(out_dir, "frames_sample_pixel.npy"), pix.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
 def host_cores() -> int:
     """Cores the CPU arm may use: the process's affinity mask, NOT OMP_NUM_THREADS (torchrun exports 1)."""
@@ -197,7 +228,7 @@ def run_reference(args):
     if rank != 0:
         return 0
     world = int(os.environ.get("WORLD_SIZE", "1"))
-    value, ms, cores, desc, n_s, _ = cpu_reference_run(max(args.steps, 5) if args.steps < 50 else 5, min(args.warmup, 2), budget_s=150.0)
+    value, ms, cores, desc, n_s, _ = cpu_reference_run(args.steps, min(args.warmup, 2), budget_s=150.0)
     line = {
         "impl": "reference", "metric": METRIC, "value": round(value, 3), "unit": "Msplats/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": round(ms, 3), "higher_is_better": True,
@@ -355,13 +386,19 @@ def run_cuda(args):
     barrier()
     ms_total = max(e0.elapsed_time(ev) for ev in e1)     # device time from the first frame's start to the last frame's / gather's end
     clk = clocks.stop() if rank == 0 else None
+    k_last = (args.steps - 1) % frames_in_flight
+    # the last timed step's frame, read before anything renders into that context again
+    dumped = None
+    if args.dump_outputs and world == 1:
+        dumped = read_device(plugins[k_last].frame_device_ptr, frame_bytes).reshape(1, HEIGHT, WIDTH, 4)
     # ---- multi-GPU correctness on hardware: rank 0 re-renders every rank's view locally and compares it with the
     #      gathered frames, byte for byte (outside the timed region)
     gather_ok = None
     if world > 1 and rank == 0:
         gather_ok = True
-        k_last = (args.steps - 1) % frames_in_flight
         gathered = all_frames[k_last].cpu().numpy().reshape(world, HEIGHT, WIDTH, 4)
+        if args.dump_outputs:
+            dumped = gathered
         for r in range(world):
             local = plugin.render_view(handle, settings, MultiViewSession(r, world, 0).view(WIDTH, HEIGHT), fmt="rgba8_srgb")
             gather_ok = gather_ok and bool(np.array_equal(local, gathered[r]))
@@ -375,15 +412,6 @@ def run_cuda(args):
     gather_ce = gather_direct = None
     peer_ready = False
     if world > 1:
-        import ctypes as C
-
-        def read_root(ptr, nbytes):
-            got = np.empty(nbytes, np.uint8)
-            cu = C.CDLL("libcuda.so.1")
-            cu.cuMemcpyDtoH_v2.argtypes = [C.c_void_p, C.c_uint64, C.c_size_t]
-            assert cu.cuMemcpyDtoH_v2(got.ctypes.data_as(C.c_void_p), C.c_uint64(ptr), got.size) == 0
-            return got
-
         def agree(ok: bool) -> bool:
             t_ = torch.tensor([1 if ok else 0], device="cuda", dtype=torch.int32)
             dist.all_reduce(t_, op=dist.ReduceOp.MIN)
@@ -433,7 +461,7 @@ def run_cuda(args):
             sig_ok = use_signal[0]
             if rank == 0 and sig_ok:
                 for k in range(frames_in_flight):
-                    words = read_root(sessions[k].peer_flags_ptr(), 4 * world).view(np.uint32)
+                    words = read_device(sessions[k].peer_flags_ptr(), 4 * world).view(np.uint32)
                     sig_ok = sig_ok and bool(np.all(words == np.uint32(sessions[k]._peer_seq & 0xFFFFFFFF)))
             use_signal[0] = agree(sig_ok)
             barrier()
@@ -457,7 +485,7 @@ def run_cuda(args):
             got = None
             if rank == 0 and use_signal[0]:
                 # read BEFORE any host barrier: the device-side wait alone has established that all frames are there
-                got = read_root(sessions[k_last]._peer_ptr.value, world * frame_bytes)
+                got = read_device(sessions[k_last]._peer_ptr.value, world * frame_bytes)
             barrier()
             leg_ms = max(c0.elapsed_time(ev) for ev in c1) / args.steps
             t_ = torch.tensor([leg_ms], device="cuda")
@@ -466,7 +494,7 @@ def run_cuda(args):
             leg_ok = None
             if rank == 0:
                 if got is None:
-                    got = read_root(sessions[k_last]._peer_ptr.value, world * frame_bytes)
+                    got = read_device(sessions[k_last]._peer_ptr.value, world * frame_bytes)
                 got = got.reshape(world, HEIGHT, WIDTH, 4)
                 leg_ok = True
                 for r in range(world):
@@ -662,6 +690,8 @@ def run_cuda(args):
         "gathered_frames_verified": gather_ok, "gather_nccl": gather_nccl, "gather_ce": gather_ce, "gather_direct": gather_direct,
         "raw_scale_1": raw, "clocks": clk,
     }
+    if dumped is not None:
+        dump_frames(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
     for se in sessions:
         se.destroy()
@@ -677,7 +707,14 @@ def main():
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the frames of the last timed step to DIR/*.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm renders a sample of the cloud sized from its own timing, "
+                 "so its output is not comparable from run to run")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)

@@ -107,3 +107,38 @@ def test_bench_arms_on_a_box_without_a_gpu():
     if not torch.cuda.is_available():
         r = subprocess.run([sys.executable, "bench.py", "--steps", "1"], cwd=root, capture_output=True, text=True, timeout=600)
         assert r.returncode != 0 and "no CUDA device" in (r.stderr + r.stdout)
+
+
+def test_bench_steps_set_the_timed_frames():
+    """--steps is the number of timed frames of either arm; a run without any is refused."""
+    import json, subprocess, sys
+    root = os.path.join(os.path.dirname(__file__), "..")
+    r = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--steps", "2", "--warmup", "3"], cwd=root,
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and "best of 2 frames" in line["cpu_baseline"]["sample"]
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = subprocess.run([sys.executable, "bench.py", *bad], cwd=root, capture_output=True, text=True, timeout=300)
+        assert r.returncode == 2, r.stderr[-2000:]
+
+
+def test_bench_dump_frames_full_and_sampled(tmp_path, monkeypatch):
+    """--dump-outputs writes the frames whole while they fit the size limit, else the same seeded pixel sample of every
+    view, identical from run to run; all of it float32 / float64 within the limit."""
+    import bench
+
+    frames = np.random.default_rng(1).integers(0, 256, (3, 40, 64, 4), dtype=np.uint8)
+    bench.dump_frames(str(tmp_path / "full"), frames)
+    assert os.listdir(tmp_path / "full") == ["frames.npy"]
+    got = np.load(tmp_path / "full" / "frames.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, frames)
+    limit = 4096 + 20_000
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", limit)
+    for d in ("a", "b"):
+        bench.dump_frames(str(tmp_path / d), frames)
+        assert sum(os.path.getsize(tmp_path / d / f) for f in os.listdir(tmp_path / d)) <= limit
+    sample, pix = np.load(tmp_path / "a" / "frames_sample.npy"), np.load(tmp_path / "a" / "frames_sample_pixel.npy")
+    assert sample.dtype == np.float32 and pix.dtype == np.float64 and sample.shape == (3, len(pix), 4) and len(pix) > 100
+    assert np.array_equal(sample, frames.reshape(3, -1, 4)[:, pix.astype(np.int64)])
+    assert np.array_equal(sample, np.load(tmp_path / "b" / "frames_sample.npy"))
